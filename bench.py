@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # product arm (one rank per GPU under torchrun for N>1)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's own training step on the host cores, rank 0 only
+    python bench.py ... --dump-outputs DIR                   # also write what the last timed training step computed, DIR/<name>.npy
 
 Headline (the half of BASELINE.json's metric that north_star sets its targets on): **train rays/s (fwd+bwd)** on configs[2] --
 ScanNet scene0241_01-shaped hybrid training step, 640x480 frames, 4096-ray batch (8x8 dilated patches of 8x8), 8 reference-view
@@ -117,6 +118,35 @@ class ClockSampler:
         hot = [x for x in sm if x >= 0.6 * max(sm)] if sm else []
         return {"sm_mhz": hot[len(hot) // 2] if hot else None, "sm_max_mhz": float(self.rows[0][1]) if self.rows[0][1].replace(".", "").isdigit() else None,
                 "reasons": reasons, "samples": len(self.rows)}
+
+
+DUMP_POINT_ROWS = 1 << 16       # rows of the point tables --dump-outputs writes: a fixed sample (seed 0) of the 2M points
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_train_outputs(out_dir, net, loss, n_valid):
+    """--dump-outputs: what the last timed training step leaves its caller, as DIR/<name>.npy (float32, counts and row ids float64):
+    the loss and valid-ray count train_step returns, every trained network parameter after the optimiser step, and of the trained
+    per-point tables the rows of DUMP_POINT_ROWS points.  The inputs are seeded, so two builds can be compared output for output."""
+    arrays = {"loss": loss.detach().float().cpu().numpy(), "valid_rays": n_valid.detach().double().cpu().numpy()}
+    rows = None
+    for name, p in net.named_parameters():
+        if not p.requires_grad:
+            continue
+        t = p.detach()
+        if name.startswith("neural_points."):
+            t = t.reshape(-1, t.shape[-1])                                   # (1, N, C) or (N, C) -> (N, C)
+            if rows is None:
+                rows = np.sort(np.random.default_rng(0).choice(t.shape[0], size=min(t.shape[0], DUMP_POINT_ROWS), replace=False))
+                arrays["neural_points.sample_rows"] = rows.astype(np.float64)
+            t = t.index_select(0, torch.from_numpy(rows).to(t.device))
+        arrays[name] = t.float().cpu().numpy()
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes > {DUMP_MAX_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ======================================================================================================================
@@ -340,7 +370,13 @@ def main():
     ap.add_argument("--no-render", action="store_true", help="skip the configs[1] full-frame render (N = 1)")
     ap.add_argument("--no-large", action="store_true", help="skip configs[4] (8M points)")
     ap.add_argument("--no-extras", action="store_true", help="skip configs[3] (blur) and the reference_gpu leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="product arm: write what the last timed training step computed to DIR/<name>.npy "
+                                                          "(rank 0 writes; the ranks' parameters are identical after the all-reduce)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "product":
+        ap.error("--dump-outputs applies to the product arm only")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
     local = int(os.environ.get("LOCAL_RANK", 0))
@@ -356,11 +392,14 @@ def main():
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     pk = peaks()
-    steps, warmup = max(3, args.steps), max(3, args.warmup)
+    steps, warmup = args.steps, max(3, args.warmup)
+    dump = None
+    if args.dump_outputs and rank == 0:
+        dump = lambda net, loss, n_valid: dump_train_outputs(args.dump_outputs, net, loss, n_valid)
 
     # ---------------------------------------------------------------- headline: configs[2] training step
     with ClockSampler(local) as clk:
-        tr = benchmarks.train_step_benchmark(dev, steps=steps, warmup=warmup, world=world, rank=rank, stage_split=(world == 1))
+        tr = benchmarks.train_step_benchmark(dev, steps=steps, warmup=warmup, world=world, rank=rank, stage_split=(world == 1), capture=dump)
     roofs = train_kernel_rooflines(tr, pk) if world == 1 else []
     top = max(roofs, key=lambda r: r["ms"]) if roofs else None
     # whole-step roofline (SURVEY 8d) against fwd+bwd time: backward on the f16 pipe like the forward (3 bf16 MMAs per product)

@@ -64,10 +64,12 @@ def _device_max(ms: float, dev, world: int) -> float:
 
 def train_step_benchmark(dev, steps: int = 5, warmup: int = 3, world: int = 1, points: int = 2_000_000, views: int = 8,
                          rank: int = 0, stage_split: bool = True, prefetch: bool = True, size=(6.0, 5.0, 3.0), H: int = 480, W: int = 640,
-                         max_o: int = 1_000_000, e2e: bool = True, workload: str = TRAIN_WORKLOAD) -> Dict:
+                         max_o: int = 1_000_000, e2e: bool = True, workload: str = TRAIN_WORKLOAD, capture=None) -> Dict:
     """One training step = forward + loss + backward (+ NCCL gradient all-reduce when world > 1) + both Adam steps, through
     parallel.train_step, on this rank's own 4096-ray raster; the next step's voxel query is software-pipelined one step ahead
     (`prefetch`).  `steps` steps are timed as ONE region between barriers (CUDA events, L2 flushed between steps), max over ranks.
+    `capture(net, loss, n_valid)`, if given, is called once after the timed steps, before any later step changes the model, with
+    what the last timed step returned and the model it updated.
     Returns a dict; 'value' = rays of ALL ranks / that time."""
     import torch.distributed as dist
     from . import parallel
@@ -95,12 +97,18 @@ def train_step_benchmark(dev, steps: int = 5, warmup: int = 3, world: int = 1, p
             torch.cuda.synchronize()
 
     # at least one pass over the whole frame set: every frame has its own valid-sample count, i.e. its own activation sizes, and the
-    # caching allocator serves a new size with a cudaMalloc (a device synchronisation) the first time it sees it
-    for _ in range(max(warmup, FRAME_SET + 1)):
+    # caching allocator serves a new size with a cudaMalloc (a device synchronisation) the first time it sees it.
+    # The barrier comes BEFORE the last warm-up step: the timed region then starts behind issued work, as every step of a training
+    # run does, and not on an idle device that waits for the host to issue its first launches (a fixed gap that a window of few
+    # steps would count as step time)
+    for _ in range(max(warmup, FRAME_SET + 1) - 1):
         cur, nx = next_pair()
         parallel.train_step(net, cur, opts, next_frame_shard=nx if prefetch else None)
     parallel.flush_pending(net)
     barrier()
+    cur, nx = next_pair()
+    parallel.train_step(net, cur, opts, next_frame_shard=nx if prefetch else None)
+    parallel.flush_pending(net)
     ops.LAUNCHES = 0
     s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     import time as _time
@@ -109,7 +117,7 @@ def train_step_benchmark(dev, steps: int = 5, warmup: int = 3, world: int = 1, p
     for _ in range(steps):
         flush.zero_()
         cur, nx = next_pair()
-        loss, _ = parallel.train_step(net, cur, opts, next_frame_shard=nx if prefetch else None)
+        loss, n_valid = parallel.train_step(net, cur, opts, next_frame_shard=nx if prefetch else None)
     parallel.flush_pending(net)
     e.record()
     host_ms = (_time.perf_counter() - t_host) / steps * 1e3           # time the HOST needs to issue a step (no synchronisation in the loop)
@@ -117,6 +125,8 @@ def train_step_benchmark(dev, steps: int = 5, warmup: int = 3, world: int = 1, p
     launches = ops.LAUNCHES
     ms_local = s.elapsed_time(e) / steps
     ms_step = _device_max(ms_local, dev, world)
+    if capture is not None:
+        capture(net, loss, n_valid)
     res = {"metric": "train rays/s (fwd+bwd)", "value": world * R / (ms_step * 1e-3), "unit": "rays/s", "ms_per_step": ms_step,
            "rays_per_step_per_gpu": R, "points": points, "views": views, "loss": float(loss), "launches_per_step": launches // steps,
            "host_issue_ms_per_step": host_ms, "frame_set": FRAME_SET,
@@ -155,13 +165,17 @@ def train_step_benchmark(dev, steps: int = 5, warmup: int = 3, world: int = 1, p
         loss_host = torch.zeros(steps + 2).pin_memory()
         cur = use(up())
         nxt_fe = up()
-        for _ in range(2):
+        def warm_step():
+            nonlocal cur, nxt_fe
             n2 = use(nxt_fe)
             nxt_fe = up()                               # two steps ahead of its first use on the main stream
             parallel.train_step(net, cur, opts, next_frame_shard=n2 if prefetch else None)
             cur = n2
+        warm_step()
         parallel.flush_pending(net)
         barrier()
+        warm_step()                                     # as above: the timed region starts behind the last warm-up step's work
+        parallel.flush_pending(net)
         s.record()
         for i in range(steps):
             flush.zero_()

@@ -2,6 +2,8 @@
 kernels, compiled from the reference source into oracle/_ref/ (oracle/build_ref_query_cubin.py) and
 launched here through cuda.bindings.  This is what pins the query oracle (north_star: "the
 reference pycuda kernel on the same box")."""
+import os
+
 import numpy as np
 import pytest
 import torch
@@ -9,6 +11,7 @@ import torch
 from helpers import cuda
 from hybridneuralrendering_b200 import make_opt
 from hybridneuralrendering_b200 import synthetic as syn
+from oracle import build_ref_query_cubin as rb
 from oracle import query_oracle as qo
 from oracle import ref_query_runner as rq
 
@@ -27,7 +30,12 @@ def _canon(p):
 @pytest.mark.parametrize("kind,N,seed", [("lego", 60000, 0), ("room", 80000, 1)])
 def test_product_and_oracle_match_reference_kernels(kind, N, seed):
     if not rq.available():
-        pytest.fail("oracle/_ref/ref_query_k8.cubin missing: run __graft_entry__.build() where /root/reference exists")
+        # the kernels are compiled from the original project's source, which the repository does not contain: without that source
+        # there is nothing to compare with; with it, a missing cubin means its build failed
+        if not os.path.isfile(rb.SRC):
+            pytest.skip(f"original project's query source {rb.SRC} not found: set HNR_REFERENCE_ROOT to a checkout of it and run "
+                        "__graft_entry__.build()")
+        pytest.fail(f"{rq.CUBIN} missing although {rb.SRC} exists: run __graft_entry__.build() (it reports why the build failed)")
     from hybridneuralrendering_b200 import lighting_fast_querier
     if kind == "lego":
         xyz, fr, opt = syn.lego_scene(N, seed), syn.lego_frame(H=40, W=40, V=1, seed=seed), make_opt("lego")
