@@ -235,7 +235,8 @@ def train_step(net, frame_shard: Dict[str, torch.Tensor], optimizers: Sequence[t
     gradients, image-branch tail: ops.defer_weight_gradients) are issued; the small MLP bucket is reduced on its own communicator
     (small_bucket_group) and its optimiser stepped at once; the all-reduce of the point tables is left in flight
     and the optimiser(s) that own those tables step at the LAST possible moment -- inside the next forward, after its query and
-    pyramid but before the first kernel that reads the tables (`net.before_point_read`), or at flush_pending(net).
+    pyramid but before the first kernel that reads the tables (`net.before_point_read`), or at flush_pending(net).  That deferred
+    step consumes the previous step's gradients, so the gradients are zeroed after the forward and flush_pending(net), not before.
     `next_frame_shard`: the shard of the NEXT step, if known -- its voxel query is enqueued before this step's backward pass so
     that the next forward does not stall at the query's read-back (NeuralPointsRayMarching.prefetch_query)."""
     from . import ops
@@ -256,10 +257,12 @@ def train_step(net, frame_shard: Dict[str, torch.Tensor], optimizers: Sequence[t
             raise NotImplementedError("data-parallel training with the patch drop needs whole (PN*PS)^2-ray rasters per rank: the reference's "
                                       "drop positions (point_aggregators.py:1222-1237) index the raster of ONE batch; give every rank its "
                                       "own raster instead of slicing one with shard_frame")
-    for o in optimizers:
-        o.zero_grad(set_to_none=True)
     out = net(**frame_shard)                        # a deferred point update of the previous step is applied inside (before_point_read)
     flush_pending(net)                               # ... or here, if the forward had nothing to read (no kept ray)
+    # zeroed only now: the deferred point-table step above reads the previous step's all-reduced gradients, and an optimiser skips a
+    # parameter whose grad is None.  The forward produces no gradients, so zeroing after it changes nothing for the other parameters
+    for o in optimizers:
+        o.zero_grad(set_to_none=True)
     mark("forward_end")
     n_local = (out["ray_mask"] > 0).sum()
     scale = n_global = None

@@ -87,8 +87,17 @@ def test_train_step_gradients_match_oracle():
     ts = net.neural_points.querier.candidate_ts(R, 0.1, 8.0, "cuda")       # the jittered draw the forward will repeat
     torch.cuda.set_rng_state(st)
     out = net(**_frame_cuda(fr))
+    mask = check_gradients_vs_oracle(net, out, fr, ts, P, dict(xyz=xyz, **att), opt)
+    full = fill_invalid(out, cuda(fr["bg_color"]), net.last_extras.ray_ids)
+    assert full["coarse_raycolor"].shape == (1, R, 3)
+    assert_close(full["coarse_raycolor"][:, ~mask], torch.ones_like(full["coarse_raycolor"][:, ~mask]), 0, 0)
+
+
+def check_gradients_vs_oracle(net, out, fr, ts, P, pts, opt):
+    """backward of the kink-masked training loss from the forward `out` of `net` (frame `fr`, candidate parameters `ts`), compared with
+    the fp64 oracle at aggregator parameters P and point attributes `pts`: the loss and every gradient.  Returns the ray mask."""
+    R = fr["raydir"].shape[1]
     mask = out["ray_mask"][0] > 0
-    pts = dict(xyz=xyz, **att)
     q = po.query(pts, fr, opt, ts.cpu().numpy().reshape(R, -1))
     np.testing.assert_array_equal(out["ray_mask"].cpu().numpy(), q["ray_mask"])
     xy, delta = _product_projections(net, fr, q["sample_loc_w"])
@@ -122,9 +131,7 @@ def test_train_step_gradients_match_oracle():
         assert_close(p.grad, r, RTOL, grad_atol(r), k)
         n += 1
     assert n >= 40
-    full = fill_invalid(out, cuda(fr["bg_color"]), net.last_extras.ray_ids)
-    assert full["coarse_raycolor"].shape == (1, R, 3)
-    assert_close(full["coarse_raycolor"][:, ~mask], torch.ones_like(full["coarse_raycolor"][:, ~mask]), 0, 0)
+    return mask
 
 
 def test_fused_training_forward_equals_layered_training_forward():

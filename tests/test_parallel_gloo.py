@@ -92,6 +92,115 @@ def test_prescaled_overlapped_allreduce_matches_full_batch_gradients(tmp_path):
             np.testing.assert_allclose(g.numpy(), ref.numpy(), rtol=1e-5, atol=1e-8)
 
 
+class _NoDefer:
+    """stand-in for ops.defer_weight_gradients (whose runner needs CUDA streams): nothing is parked, so there is nothing to run"""
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        return False
+
+    def run(self):
+        pass
+
+
+class _ToyNet(torch.nn.Module):
+    """the parts of NeuralPointsRayMarching that train_step relies on: a point table over the deferred-step threshold (32768 x 39
+    fp32 = 5.1 MB > 4 MB), a small "MLP", and the `before_point_read` hook, run before the table is read"""
+
+    def __init__(self):
+        super().__init__()
+        g = torch.Generator().manual_seed(0)
+        self.table = torch.nn.Parameter(torch.randn(_TABLE_ROWS, 39, generator=g))
+        self.w1 = torch.nn.Parameter(torch.randn(39, 16, generator=g) * 0.1)
+        self.w2 = torch.nn.Parameter(torch.randn(16, 3, generator=g) * 0.1)
+        self.before_point_read = None
+
+    def forward(self, idx, valid, **_):
+        if self.before_point_read is not None:
+            cb, self.before_point_read = self.before_point_read, None
+            cb()
+        m = valid.bool()
+        color = torch.tanh(self.table[idx[m]] @ self.w1) @ self.w2
+        return {"coarse_raycolor": color[None], "ray_mask": valid.to(torch.int8)[None]}
+
+
+_TABLE_ROWS = 32768
+_STEPS = 3
+
+
+def _toy_optimizers(net):
+    """the two Adam groups of benchmarks.make_optimizers (network lr 5e-4, point table lr 2e-3), as torch.optim.Adam"""
+    return [torch.optim.Adam([net.w1, net.w2], lr=5e-4), torch.optim.Adam([net.table], lr=2e-3)]
+
+
+def _toy_raster(step, rank, R=256):
+    """rank `rank`'s own raster of training step `step`"""
+    g = torch.Generator().manual_seed(1000 + 10 * step + rank)
+    idx = torch.randint(0, _TABLE_ROWS, (R,), generator=g)
+    gt = torch.rand(1, R, 3, generator=g)
+    valid = torch.rand(R, generator=g) > 0.3
+    return {"idx": idx, "valid": valid, "gt_image": gt}
+
+
+def _worker_train_steps(rank, world, port, out_dir):
+    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), HNR_SMALL_BUCKET="nccl")
+    from hybridneuralrendering_b200 import ops
+    ops.defer_weight_gradients = _NoDefer
+    dist.init_process_group("gloo", rank=rank, world_size=world)
+    net = _ToyNet()
+    opts = _toy_optimizers(net)
+    losses, n_globals = [], []
+    for k in range(_STEPS):
+        loss, n_global = parallel.train_step(net, _toy_raster(k, rank), opts)
+        losses.append(float(loss))
+        n_globals.append(float(n_global))
+    parallel.flush_pending(net)
+    torch.save({"params": {n: p.detach().clone() for n, p in net.named_parameters()},
+                "steps": {n: int(opts[i].state[p]["step"]) for i, n, p in ((1, "table", net.table), (0, "w1", net.w1), (0, "w2", net.w2))},
+                "losses": losses, "n_global": n_globals}, os.path.join(out_dir, f"r{rank}.pt"))
+    dist.destroy_process_group()
+
+
+def test_train_step_trains_point_tables_across_steps(tmp_path):
+    """three data-parallel train_steps on two ranks, then flush_pending, against one process that steps Adam on the n_valid-weighted
+    mean of both rasters' gradients every step.  The point table's optimiser step is deferred into the next forward; it must see the
+    gradients of the step before (it was skipped when they had already been zeroed: step count 1, the table moved only at the flush)."""
+    world = 2
+    mp.spawn(_worker_train_steps, args=(world, _free_port(), str(tmp_path)), nprocs=world, join=True)
+    outs = [torch.load(os.path.join(tmp_path, f"r{r}.pt")) for r in range(world)]
+    net = _ToyNet()
+    opts = _toy_optimizers(net)
+    start = net.table.detach().clone()
+    for k in range(_STEPS):
+        for o in opts:
+            o.zero_grad(set_to_none=True)
+        rasters = [_toy_raster(k, r) for r in range(world)]
+        n = [r["valid"].sum().to(torch.float32) for r in rasters]
+        n_global = n[0] + n[1]
+        for r, fr in enumerate(rasters):
+            # the same float32 scale train_step applies to each rank's loss (global_mean_scale)
+            out = net(**fr)
+            loss = torch.nn.functional.mse_loss(out["coarse_raycolor"], fr["gt_image"][:, fr["valid"]])
+            (loss * (n[r] / n_global)).backward()
+        for o in opts:
+            o.step()
+        for r in range(world):
+            assert outs[r]["n_global"][k] == float(n_global)
+    for r in range(world):
+        assert outs[r]["steps"] == {"table": _STEPS, "w1": _STEPS, "w2": _STEPS}
+        for name, p in net.named_parameters():
+            # both sides run the same float32 torch arithmetic; rtol 1e-6 leaves room for the all-reduce summing the two ranks'
+            # gradients in another order than the reference's accumulation (atol: 1e-6 of the smaller learning rate, for entries near 0)
+            np.testing.assert_allclose(outs[r]["params"][name].numpy(), p.detach().numpy(), rtol=1e-6, atol=5e-10, err_msg=name)
+    for name in outs[0]["params"]:
+        assert torch.equal(outs[0]["params"][name], outs[1]["params"][name]), name
+    # every row a ray of any step read has moved (with the update skipped, only the rows of the last step moved, at the flush)
+    touched = torch.cat([_toy_raster(k, r)["idx"][_toy_raster(k, r)["valid"]] for k in range(_STEPS) for r in range(world)]).unique()
+    assert bool((outs[0]["params"]["table"][touched] != start[touched]).any(dim=1).all())
+
+
 def test_shard_patches_partition():
     for R, world in ((3136, 8), (4096, 3), (64, 4)):
         spans = [parallel.shard_patches(R, 64, r, world) for r in range(world)]
