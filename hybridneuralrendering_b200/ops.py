@@ -951,11 +951,33 @@ class CompositeFn(torch.autograd.Function):
 # --------------------------------------------------------------------------------------------
 # blur
 # --------------------------------------------------------------------------------------------
+# The blur kernels index the raster from patch_num and patch_size alone, so a tensor of the wrong shape would be read and
+# written out of bounds: the shapes are checked on the host before anything is launched.
+def _check_raster(name: str, t: torch.Tensor, patch_num: int, patch_size: int) -> None:
+    rows = (patch_num * patch_size) ** 2
+    if t.dim() != 2 or t.shape[0] != rows or t.shape[1] != 3:
+        raise ValueError(f"blur: {name} must be ((patch_num*patch_size)^2, 3) = ({rows}, 3) for patch_num {patch_num}, "
+                         f"patch_size {patch_size}; got {tuple(t.shape)}")
+
+
+def _check_kernel_bank(kernels: torch.Tensor) -> None:
+    if kernels.dim() != 3 or kernels.shape[1] != kernels.shape[2] or kernels.shape[1] % 2 == 0:
+        raise ValueError(f"blur: kernels must be (Nk, k, k) with k odd; got {tuple(kernels.shape)}")
+
+
+def _check_raw(raw: torch.Tensor, patch_num: int) -> None:
+    if raw.dim() != 2 or raw.shape[0] != patch_num * patch_num:
+        raise ValueError(f"blur: raw predictor output must have patch_num^2 = {patch_num * patch_num} rows; got {tuple(raw.shape)}")
+
+
 class BlurSelectFn(torch.autograd.Function):
     """pred, gt (S*S,3) on the patch raster; kernels (Nk,ks,ks) -> best candidate per patch."""
 
     @staticmethod
     def forward(ctx, pred, gt, kernels, patch_num: int, patch_size: int):
+        _check_raster("pred", pred, patch_num, patch_size)
+        _check_raster("gt", gt, patch_num, patch_size)
+        _check_kernel_bank(kernels)
         pred, gt, kernels = _f32c(pred), _f32c(gt), _f32c(kernels)
         require_cuda(pred, gt, kernels)
         Nk, ks = kernels.shape[0], kernels.shape[1]
@@ -986,6 +1008,8 @@ class BlurGrayFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, pred, gt, patch_num: int, patch_size: int):
+        _check_raster("pred", pred, patch_num, patch_size)
+        _check_raster("gt", gt, patch_num, patch_size)
         pred, gt = _f32c(pred), _f32c(gt)
         require_cuda(pred, gt)
         feat = torch.empty((patch_num * patch_num, 2 * patch_size * patch_size), device=pred.device, dtype=torch.float32)
@@ -1010,9 +1034,10 @@ class BlurLearnFn(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, pred, raw, patch_num: int, patch_size: int, kernel_size: int, norm_mode: int, mix_mode: int, boundary_mode: int):
+        _check_raster("pred", pred, patch_num, patch_size)
+        _check_raw(raw, patch_num)
         pred, raw = _f32c(pred), _f32c(raw)
         require_cuda(pred, raw)
-        assert raw.dim() == 2 and raw.shape[0] == patch_num * patch_num
         out = torch.empty_like(pred)
         with _launch(name="blur_learn_fwd"):
             check(lib().hnr_blur_learn_fwd(ptr(pred), ptr(raw), raw.shape[1], patch_num, patch_size, kernel_size, norm_mode, mix_mode,

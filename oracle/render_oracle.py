@@ -316,28 +316,31 @@ def ray_march(ray_dist, ray_valid, feats, bg_color=None):
 # ----------------------------------------------------------------------------------------------
 # B1: blur module
 # ----------------------------------------------------------------------------------------------
-def blur_select(pred: torch.Tensor, gt: torch.Tensor, kernels: torch.Tensor, patch_num: int, patch_size: int):
+def blur_select(pred: torch.Tensor, gt: torch.Tensor, kernels: torch.Tensor, patch_num: int, patch_size: int, select=None):
     """pred, gt (1,S*S,3) on an S x S raster of patch_num^2 patches; kernels (1,Nk,kh,kw).
-    Returns (new_pred (1,S*S,3), select_index (patch_num^2,)).  base_rendering_model.py:677-786."""
+    Returns (new_pred (1,S*S,3), select_index (patch_num^2,)).  base_rendering_model.py:677-786.
+    `select` (patch_num^2,): use these candidates instead of the argmin (tests pass the product's pick where two candidates'
+    errors tie to rounding)."""
+    cand, err = blur_candidates(pred, gt, kernels, patch_num, patch_size)
+    sel = torch.argmin(err, dim=1) if select is None else torch.as_tensor(select).long().reshape(-1)
+    best = cand[torch.arange(cand.shape[0]), :, sel]                   # (P2,3,p,p)
     S = patch_num * patch_size
+    img = best.reshape(patch_num, patch_num, 3, patch_size, patch_size).permute(2, 0, 3, 1, 4).reshape(3, S, S)
+    return img.permute(1, 2, 0).reshape(1, S * S, 3), sel
+
+
+def blur_candidates(pred: torch.Tensor, gt: torch.Tensor, kernels: torch.Tensor, patch_num: int, patch_size: int):
+    """every candidate of blur_select: (cand (P2,3,Nk+1,p,p) -- the Nk border-renormalised blurs, then the patch itself --,
+    err (P2,Nk+1) the L1 distance of each candidate to the ground truth)"""
     Nk, kh = kernels.shape[1], kernels.shape[2]
-
-    def to_patches(x):
-        x = x.reshape(S, S, 3).permute(2, 0, 1)                      # (3,S,S)
-        x = x.reshape(3, patch_num, patch_size, patch_num, patch_size)
-        return x.permute(1, 3, 0, 2, 4).reshape(patch_num * patch_num, 3, patch_size, patch_size)
-
-    xp, gp = to_patches(pred), to_patches(gt)
+    xp, gp = _blur_patches(pred, patch_num, patch_size), _blur_patches(gt, patch_num, patch_size)
     flat = xp.reshape(-1, 1, patch_size, patch_size)
     k = kernels[0].unsqueeze(1).to(flat)
     norm = F.conv2d(torch.ones_like(flat), k, padding=kh // 2)
     blurred = F.conv2d(flat, k, padding=kh // 2) / norm               # (P2*3,Nk,p,p)
     cand = torch.cat([blurred, flat], dim=1).reshape(-1, 3, Nk + 1, patch_size, patch_size)
     err = (cand - gp.unsqueeze(2)).abs().sum(dim=(1, 3, 4))            # (P2,Nk+1)
-    sel = torch.argmin(err, dim=1)
-    best = cand[torch.arange(cand.shape[0]), :, sel]                   # (P2,3,p,p)
-    img = best.reshape(patch_num, patch_num, 3, patch_size, patch_size).permute(2, 0, 3, 1, 4).reshape(3, S, S)
-    return img.permute(1, 2, 0).reshape(1, S * S, 3), sel
+    return cand, err
 
 
 # ----------------------------------------------------------------------------------------------
@@ -348,18 +351,28 @@ def learnable_blur(pred: torch.Tensor, gt: torch.Tensor, weights, patch_num: int
     """pred, gt (1,S*S,3) on the patch raster; weights = [(W,b)] * 4 of learn_blur_kernel_block (point_aggregators.py:715-749).
     Returns (new_pred (1,S*S,3), raw predictor output (N, ks^2 [+1])).  base_rendering_model.py:827-1020 with
     learnable_blur_kernel_conv=0."""
-    S, N, KK = patch_num * patch_size, patch_num * patch_num, kernel_size * kernel_size
-
-    def to_patches(x):
-        x = x.reshape(S, S, 3).permute(2, 0, 1).reshape(3, patch_num, patch_size, patch_num, patch_size)
-        return x.permute(1, 3, 0, 2, 4).reshape(N, 3, patch_size, patch_size)
-
-    xp, gp = to_patches(pred), to_patches(gt)
+    N = patch_num * patch_num
+    xp, gp = _blur_patches(pred, patch_num, patch_size), _blur_patches(gt, patch_num, patch_size)
     x = torch.cat([gp.mean(dim=1).reshape(N, -1), xp.mean(dim=1).reshape(N, -1)], dim=-1)          # :887-889
     for i, (W, b) in enumerate(weights):
         x = F.linear(x, W, b)
-        x = torch.sigmoid(x) if i == len(weights) - 1 else F.leaky_relu(x, 0.01)
-    raw = x
+        x = torch.sigmoid(x) if i == len(weights) - 1 else _act(x)
+    return learnable_blur_apply(pred, x, patch_num, patch_size, kernel_size, kernel_mode, kernel_norm, boundary_mode), x
+
+
+def _blur_patches(x, patch_num, patch_size):
+    """(1,S*S,3) patch raster -> (patch_num^2,3,p,p), patches in row-major order"""
+    S = patch_num * patch_size
+    x = x.reshape(S, S, 3).permute(2, 0, 1).reshape(3, patch_num, patch_size, patch_num, patch_size)
+    return x.permute(1, 3, 0, 2, 4).reshape(patch_num * patch_num, 3, patch_size, patch_size)
+
+
+def learnable_blur_apply(pred: torch.Tensor, raw: torch.Tensor, patch_num: int, patch_size: int, kernel_size: int = 9,
+                         kernel_mode: int = 4, kernel_norm: int = 0, boundary_mode: int = 0):
+    """the part of learnable_blur after the predictor: raw predictor output (N, ks^2 [+1]) -> per-patch kernel -> blurred
+    patch raster (1,S*S,3).  base_rendering_model.py:895-1005."""
+    S, N, KK = patch_num * patch_size, patch_num * patch_num, kernel_size * kernel_size
+    xp = _blur_patches(pred, patch_num, patch_size)
     if kernel_norm == 0:                                                                             # :895-899
         k = raw[:, :KK].view(N, 1, kernel_size, kernel_size)
         k = k / k.sum(dim=(2, 3), keepdim=True)
@@ -385,7 +398,7 @@ def learnable_blur(pred: torch.Tensor, gt: torch.Tensor, weights, patch_num: int
         raise NotImplementedError
     best = y.permute(1, 0, 2, 3)                                                                     # (N,3,p,p)
     img = best.reshape(patch_num, patch_num, 3, patch_size, patch_size).permute(2, 0, 3, 1, 4).reshape(3, S, S)
-    return img.permute(1, 2, 0).reshape(1, S * S, 3), raw
+    return img.permute(1, 2, 0).reshape(1, S * S, 3)
 
 
 def blur_predictor_params(seed: int, patch_size: int = 8, kernel_size: int = 9, kernel_mode: int = 4):

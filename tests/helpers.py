@@ -28,6 +28,22 @@ def build_aggregator(P, **opt_over):
     return agg
 
 
+def blur_predictor(params):
+    """learn_blur_kernel_block with the given [(W,b)]*4, built by the product's own aggregator so the state_dict names are the
+    checkpoint's (learn_blur_kernel_block.{0,2,4,6})."""
+    from hybridneuralrendering_b200 import PointAggregator
+    KK1, K0 = params[-1][0].shape[0], params[0][0].shape[1]
+    ks = int(np.sqrt(KK1))
+    agg = PointAggregator(make_opt(is_train=True, learnable_blur_kernel=1, learnable_blur_kernel_size=ks,
+                                   learnable_blur_patch_size=int(np.sqrt(K0 // 2)), learnable_blur_kernel_mode=4 if KK1 > ks * ks else 0)).cuda()
+    sd = {}
+    for li, (W, b) in enumerate(params):
+        sd[f"learn_blur_kernel_block.{2 * li}.weight"], sd[f"learn_blur_kernel_block.{2 * li}.bias"] = W, b
+    missing = agg.load_state_dict(sd, strict=False)
+    assert not missing.unexpected_keys
+    return agg.learn_blur_kernel_block
+
+
 def run_dropin(agg, d, g, grad=False):
     """call the drop-in forward with the gathered tensors of synthetic case (d, g)"""
     leaf = {k: cuda(g[k]).clone().requires_grad_(grad) for k in ("sampled_embedding", "sampled_color", "sampled_dir", "sampled_conf")}

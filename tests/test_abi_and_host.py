@@ -50,6 +50,43 @@ def test_product_does_not_import_oracle():
             assert "oracle" not in re.sub(r'""".*?"""', "", src, flags=re.S).replace("# ", ""), fn
 
 
+def test_blur_wrappers_reject_bad_shapes_before_launch():
+    """the blur kernels index the raster from patch_num / patch_size alone: every wrapper checks its shapes on the host (CPU
+    tensors here, so a check that came after the CUDA guard would raise RuntimeError instead)"""
+    from hybridneuralrendering_b200 import ops
+    PN, PS, KS = 2, 3, 5
+    n = (PN * PS) ** 2
+    ok, ker, raw = torch.zeros(n, 3), torch.zeros(4, KS, KS), torch.zeros(PN * PN, KS * KS + 1)
+    bad_rasters = [torch.zeros(n - 1, 3), torch.zeros(n + PS, 3), torch.zeros(n, 4), torch.zeros(n, 1), torch.zeros(n * 3),
+                   torch.zeros(1, n, 3)]
+    for bad in bad_rasters:
+        with pytest.raises(ValueError, match="pred"):
+            ops.BlurSelectFn.apply(bad, ok, ker, PN, PS)
+        with pytest.raises(ValueError, match="gt"):
+            ops.BlurSelectFn.apply(ok, bad, ker, PN, PS)
+        with pytest.raises(ValueError, match="pred"):
+            ops.BlurGrayFn.apply(bad, ok, PN, PS)
+        with pytest.raises(ValueError, match="gt"):
+            ops.BlurGrayFn.apply(ok, bad, PN, PS)
+        with pytest.raises(ValueError, match="pred"):
+            ops.BlurLearnFn.apply(bad, raw, PN, PS, KS, 0, 4, 1)
+    with pytest.raises(ValueError, match="pred"):                # the raster of a 1-patch-larger grid
+        ops.BlurSelectFn.apply(torch.zeros(((PN + 1) * PS) ** 2, 3), torch.zeros(((PN + 1) * PS) ** 2, 3), ker, PN, PS)
+    for bad in (torch.zeros(4, KS, KS - 1), torch.zeros(4, KS - 1, KS - 1), torch.zeros(KS, KS), torch.zeros(1, 4, KS, KS)):
+        with pytest.raises(ValueError, match="kernels"):
+            ops.BlurSelectFn.apply(ok, ok, bad, PN, PS)
+    for bad in (torch.zeros(PN * PN - 1, KS * KS + 1), torch.zeros(PN * PN + 1, KS * KS + 1), torch.zeros(PN * PN * (KS * KS + 1))):
+        with pytest.raises(ValueError, match="raw"):
+            ops.BlurLearnFn.apply(ok, bad, PN, PS, KS, 0, 4, 1)
+    # well-formed CPU tensors pass the shape checks and stop at the CUDA guard
+    with pytest.raises(RuntimeError, match="CUDA"):
+        ops.BlurSelectFn.apply(ok, ok, ker, PN, PS)
+    with pytest.raises(RuntimeError, match="CUDA"):
+        ops.BlurGrayFn.apply(ok, ok, PN, PS)
+    with pytest.raises(RuntimeError, match="CUDA"):
+        ops.BlurLearnFn.apply(ok, raw, PN, PS, KS, 0, 4, 1)
+
+
 def test_aggregator_state_dict_matches_reference_layout():
     from hybridneuralrendering_b200 import PointAggregator, make_opt
     from oracle import render_oracle as ro

@@ -3,7 +3,7 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import T, assert_close, cuda, grad_atol, load_golden
+from helpers import T, assert_close, blur_predictor, cuda, grad_atol, load_golden
 from oracle import render_oracle as ro
 
 pytestmark = pytest.mark.gpu
@@ -102,22 +102,6 @@ def test_blur_module_method_dropin_shipped_shape():
     assert_close(m.output["coarse_raycolor"], ref, RTOL, 1e-6)
 
 
-def _blur_predictor(params):
-    """learn_blur_kernel_block with the given [(W,b)]*4, built by the product's own aggregator so the state_dict names are the
-    checkpoint's (learn_blur_kernel_block.{0,2,4,6})."""
-    from hybridneuralrendering_b200 import PointAggregator, make_opt
-    KK1, K0 = params[-1][0].shape[0], params[0][0].shape[1]
-    ks = int(np.sqrt(KK1))
-    agg = PointAggregator(make_opt(is_train=True, learnable_blur_kernel=1, learnable_blur_kernel_size=ks,
-                                   learnable_blur_patch_size=int(np.sqrt(K0 // 2)), learnable_blur_kernel_mode=4 if KK1 > ks * ks else 0)).cuda()
-    sd = {}
-    for li, (W, b) in enumerate(params):
-        sd[f"learn_blur_kernel_block.{2 * li}.weight"], sd[f"learn_blur_kernel_block.{2 * li}.bias"] = W, b
-    missing = agg.load_state_dict(sd, strict=False)
-    assert not missing.unexpected_keys
-    return agg.learn_blur_kernel_block
-
-
 def test_learnable_blur_golden_fwd_bwd():
     """N3 (SURVEY 8f): learnable_blur_update_output through the drop-in method body vs outputs and gradients of the unmodified
     reference (tests/golden/blur_learn.npz), every norm / mode / boundary branch of the fixture."""
@@ -126,7 +110,7 @@ def test_learnable_blur_golden_fwd_bwd():
     G = load_golden("blur_learn")
     PN, PS, KS = [int(v) for v in G["meta"]]
     for ci, (mode, norm, bmode) in enumerate(G["cases"].tolist()):
-        blk = _blur_predictor(ro.blur_predictor_params(100 + ci, PS, KS, mode))
+        blk = blur_predictor(ro.blur_predictor_params(100 + ci, PS, KS, mode))
         pred = cuda(G["pred"]).clone().requires_grad_(True)
         opt = types.SimpleNamespace(learnable_blur_kernel_size=KS, learnable_blur_kernel_mode=mode, learnable_blur_kernel_norm=norm,
                                     learnable_blur_kernel_conv=0, boundary_mode=bmode)
@@ -151,11 +135,11 @@ def test_learnable_blur_shipped_shape_vs_oracle():
     P = ro.blur_predictor_params(7, PS, KS, 4)
     pred, gt = T(rng.random((1, (PN * PS) ** 2, 3), dtype=np.float32)), T(rng.random((1, (PN * PS) ** 2, 3), dtype=np.float32))
     ref, raw_ref = ro.learnable_blur(pred, gt, P, PN, PS, KS, 4, 0, 1)
-    out, raw = learnable_blur(pred.cuda(), gt.cuda(), _blur_predictor(P), PN, PS, KS, 4, 0, 1)
+    out, raw = learnable_blur(pred.cuda(), gt.cuda(), blur_predictor(P), PN, PS, KS, 4, 0, 1)
     assert_close(raw, raw_ref, RTOL, 1e-6)
     assert_close(out, ref, RTOL, 1e-6)
     P[-1][1][-1] = -1e4                          # sigmoid -> 0: kernel = identity
-    out, raw = learnable_blur(pred.cuda(), gt.cuda(), _blur_predictor(P), PN, PS, KS, 4, 0, 1)
+    out, raw = learnable_blur(pred.cuda(), gt.cuda(), blur_predictor(P), PN, PS, KS, 4, 0, 1)
     assert float(raw[:, -1].abs().max()) == 0.0
     assert_close(out, pred, 1e-6, 1e-7)
 
