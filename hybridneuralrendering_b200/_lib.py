@@ -100,7 +100,7 @@ _SIGS = {
     "hnr_img_sum_views": (C.c_int, [vp, i64, i64, i64, vp, i64, vp]),
     "hnr_chain_bwd_f16": (C.c_int, [C.c_int, C.POINTER(i64), C.POINTER(i64), i64, C.c_int, vp, i64, vp, i64, C.POINTER(vp), C.POINTER(vp), vp,
                                     C.POINTER(i64), vp, i64, i64, vp]),
-    "hnr_train_loss": (C.c_int, [vp, vp, vp, i64, vp, i64, f32c, f32c, vp, vp, vp, vp]),
+    "hnr_train_loss": (C.c_int, [vp, vp, vp, i64, vp, i64, f32c, f32c, vp, vp, vp, vp, vp]),
     "hnr_pyramid_fwd": (C.c_int, [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), i64, i64, i64, vp]),
     "hnr_pyramid_bwd": (C.c_int, [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), i64, i64, i64, vp]),
     "hnr_pack_job_bytes": (i64, []),

@@ -693,9 +693,13 @@ def _x0_cols(dev):
 # --------------------------------------------------------------------------------------------
 # image branch
 # --------------------------------------------------------------------------------------------
+TRAIN_LOSS_PARTIALS = 512        # HNR_TRAIN_LOSS_PARTIALS (include/hnr.h): scratch doubles of hnr_train_loss
+
+
 class TrainLossFn(torch.autograd.Function):
-    """training loss of the hot path in one launch (csrc/loss.cu): masked MSE (+1e-6) x frame_weight + zero-one regulariser on
-    conf_coefficient; the gradients are computed by the same launch and only scaled in backward."""
+    """training loss of the hot path (csrc/loss.cu): masked MSE (+1e-6) x frame_weight + zero-one regulariser on conf_coefficient;
+    the gradients are computed by the same launch and only scaled in backward.  A second one-warp launch adds the block partials in a
+    fixed order, so the value is the same in every run."""
 
     @staticmethod
     def forward(ctx, color, confc, gt, ray_ids, frame_weight: float, zero_one_weight: float):
@@ -704,12 +708,13 @@ class TrainLossFn(torch.autograd.Function):
         n_rays = color.numel() // 3
         cc = _f32c(confc) if confc is not None else None
         dev = color.device
-        loss = torch.zeros((), device=dev, dtype=torch.float32)
+        loss = torch.empty((), device=dev, dtype=torch.float32)
+        partials = torch.empty(TRAIN_LOSS_PARTIALS, device=dev, dtype=torch.float64)
         d_color = torch.empty_like(color)
         d_cc = torch.empty_like(cc) if cc is not None else None
-        with _launch(name="train_loss"):
+        with _launch(2, name="train_loss"):
             check(lib().hnr_train_loss(ptr(color), ptr(gt2), ptr(ray_ids), n_rays, ptr(cc), cc.numel() if cc is not None else 0, float(frame_weight),
-                                       float(zero_one_weight), ptr(loss), ptr(d_color), ptr(d_cc), stream()), "train_loss")
+                                       float(zero_one_weight), ptr(loss), ptr(partials), ptr(d_color), ptr(d_cc), stream()), "train_loss")
         ctx.save_for_backward(d_color, d_cc if d_cc is not None else torch.empty(0, device=dev))
         ctx.has_cc = cc is not None
         return loss

@@ -248,10 +248,13 @@ int hnr_img_sum_views(const void* img, int64_t C, int64_t Nv, int64_t V, float* 
 int hnr_chain_bwd_f16(int nlayer, const int64_t* Np, const int64_t* N, int64_t NX, int act_top, const float* dY, int64_t lddy,
                       const float* Ytop, int64_t ldyt, const void* const* gimg, void* const* dzimg, const void* wpackT,
                       const int64_t* w_off, float* dX, int64_t ldx, int64_t M, void* stream);
-/* Training loss in one launch (csrc/loss.cu): masked MSE (+1e-6) x frame_weight + zero-one regulariser on conf_coefficient
- * (models/base_rendering_model.py:1114-1118, :1205-1206, :1229-1240); value and both gradients.  loss must be zeroed by the caller. */
+/* Training loss (csrc/loss.cu): masked MSE (+1e-6) x frame_weight + zero-one regulariser on conf_coefficient
+ * (models/base_rendering_model.py:1114-1118, :1205-1206, :1229-1240); value (written to loss) and both gradients.  The per-block
+ * partial sums go through `partials` (HNR_TRAIN_LOSS_PARTIALS doubles of scratch) and are added in a fixed order: the value is the
+ * same in every run. */
+#define HNR_TRAIN_LOSS_PARTIALS 512
 int hnr_train_loss(const float* color, const float* gt, const int32_t* ray_ids, int64_t n_rays, const float* confc, int64_t n_conf,
-                   float frame_weight, float zero_one_weight, float* loss, float* d_color, float* d_confc, void* stream);
+                   float frame_weight, float zero_one_weight, float* loss, double* partials, float* d_color, float* d_confc, void* stream);
 /* Feature pyramid of the image branch (csrc/pyramid.cu): the six 3x3 convolutions + LeakyReLU of aux_block_s1/s2/s3
  * (models/aggregators/point_aggregators.py:598-630, :1047-1063), exact fp32, NHWC, forward and backward.  w/b: six torch-layout
  * (Cout,Cin,3,3) / (Cout) tensors; act: the six activated outputs (act[1], act[3], act[5] are the levels the lookup reads);

@@ -248,23 +248,11 @@ def _free_port():
     return port
 
 
-def test_two_ranks_match_single_process_steps(tmp_path):
-    """parallel.train_step on 2 gloo ranks sharing this GPU (each rank its own raster; HNR_SMALL_BUCKET=nccl: no symmetric memory),
-    3 steps and flush_pending, against one process that accumulates, per step, the backward of training_loss x n_r / (n_0 + n_1)
-    of both rasters and then steps both FusedAdam groups.  The point-table step is deferred into the next forward on the ranks."""
+def _reference_worker(_, out_dir):
+    """the single-process reference of test_two_ranks_match_single_process_steps, in a fresh process like the ranks: per step, the
+    backward of training_loss x n_r / (n_0 + n_1) of both rasters accumulated, then both FusedAdam groups stepped"""
+    torch.cuda.set_device(0)
     world = 2
-    ctx = mp.spawn(_rank_worker, args=(world, _free_port(), str(tmp_path)), nprocs=world, join=False)
-    try:
-        deadline = time.monotonic() + 300
-        while not ctx.join(timeout=5):
-            assert time.monotonic() < deadline, "the ranks did not finish within 300 s"
-    finally:
-        for p in ctx.processes:
-            if p.is_alive():
-                p.kill()
-            p.join()
-    outs = [torch.load(os.path.join(tmp_path, f"r{r}.pt")) for r in range(world)]
-
     opt = _opt()
     xyz, att, P = _scene()
     net = _net(opt, xyz, att, P)
@@ -273,6 +261,7 @@ def test_two_ranks_match_single_process_steps(tmp_path):
     opts = make_optimizers(net)
     named = _trainable(net)
     start = {n: p.detach().cpu().clone() for n, p in named}
+    n_global = []
     for k in range(DP_STEPS):
         for o in opts:
             o.zero_grad(set_to_none=True)
@@ -287,16 +276,45 @@ def test_two_ranks_match_single_process_steps(tmp_path):
             (training_loss(out, frames[r][k]["gt_image"]) * (n[r] / (n[0] + n[1]))).backward()
         for o in opts:
             o.step()
-        for r in range(world):
-            assert outs[r]["n_global"][k] == float(n[0] + n[1])
+        n_global.append(float(n[0] + n[1]))
+    torch.save({"params": {n: p.detach().cpu() for n, p in named}, "start": start, "n_global": n_global}, os.path.join(out_dir, "ref.pt"))
+
+
+def _run_spawned(fn, args, nprocs):
+    ctx = mp.spawn(fn, args=args, nprocs=nprocs, join=False)
+    try:
+        deadline = time.monotonic() + 300
+        while not ctx.join(timeout=5):
+            assert time.monotonic() < deadline, "the processes did not finish within 300 s"
+    finally:
+        for p in ctx.processes:
+            if p.is_alive():
+                p.kill()
+            p.join()
+
+
+def test_two_ranks_match_single_process_steps(tmp_path):
+    """parallel.train_step on 2 gloo ranks sharing this GPU (each rank its own raster; HNR_SMALL_BUCKET=nccl: no symmetric memory),
+    3 steps and flush_pending, against one process that accumulates, per step, the backward of training_loss x n_r / (n_0 + n_1)
+    of both rasters and then steps both FusedAdam groups.  The point-table step is deferred into the next forward on the ranks.
+    The reference runs in a fresh process too, so both sides start from the same process state whatever ran before in this one (the
+    noise floor of the fp32 atomics, which decides the Adam sign of the near-zero point-table gradients, otherwise follows it)."""
+    world = 2
+    _run_spawned(_rank_worker, (world, _free_port(), str(tmp_path)), world)
+    outs = [torch.load(os.path.join(tmp_path, f"r{r}.pt")) for r in range(world)]
+    _run_spawned(_reference_worker, (str(tmp_path),), 1)
+    ref = torch.load(os.path.join(tmp_path, "ref.pt"))
+    for r in range(world):
+        assert outs[r]["n_global"] == ref["n_global"]
     assert outs[0]["steps"] == outs[1]["steps"] == [DP_STEPS]
     for n_ in outs[0]["params"]:
         assert torch.equal(outs[0]["params"][n_], outs[1]["params"][n_]), n_
+    assert set(outs[0]["params"]) == set(ref["params"])
     report = []
-    _compare_params([(n_, p.cpu()) for n_, p in outs[0]["params"].items()], {n_: p.detach() for n_, p in named}, "after flush", report)
+    _compare_params(list(outs[0]["params"].items()), ref["params"], "after flush", report)
     for n_, p in outs[0]["params"].items():
         if n_.startswith("neural_points."):
-            assert int((p != start[n_])[0].any(-1).sum()) > 100, n_       # the point tables moved
+            assert int((p != ref["start"][n_])[0].any(-1).sum()) > 100, n_       # the point tables moved
     _print_report("two gloo ranks vs single process", report)
 
 

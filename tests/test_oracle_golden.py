@@ -235,3 +235,80 @@ def test_agg_train_shipped_shape_grads_match_reference():
         np.testing.assert_allclose(p.grad.numpy(), ref, rtol=2e-4, atol=1e-7 + 1e-4 * np.abs(ref).max(), err_msg=k)
         n += 1
     assert n >= 40
+
+
+def test_kernel_references_match_oracle(monkeypatch):
+    """the fp64 references of the per-kernel GPU tests (tests/helpers.py ref_*) against the oracle's own expressions on one small case:
+    pos_enc, feature_pyramid, full_res_features + the truncated pixel lookup, and the weight, MLP-input, density-head / K-sum and blend
+    expressions inside aggregate(), read off the inputs and outputs of its dense layers.  The oracle is pinned to the reference's
+    goldens above, so this ties the yardstick of tests/test_gpu_aggregate_kernels.py to them too."""
+    import helpers as h
+    dt = torch.float64
+    R, SR, K, V = 7, 6, 8, 2
+    S = R * SR
+    d = syn.render_stage_inputs(seed=5, N=300, R=R, SR=SR, K=K, V=V, H=19, W=27, empty_frac=0.3)
+    g = syn.gather_neighbours(d)
+    P = ro.random_params(seed=6, dtype=dt)
+    c = lambda a: T(a).to(dt)
+    a, b = 0.7, -0.4                                         # a world->camera rotation that is not the identity
+    rz = torch.tensor([[np.cos(a), -np.sin(a), 0], [np.sin(a), np.cos(a), 0], [0, 0, 1]], dtype=dt)
+    rx = torch.tensor([[1, 0, 0], [0, np.cos(b), -np.sin(b)], [0, np.sin(b), np.cos(b)]], dtype=dt)
+    rw2c = rz @ rx
+    taps, lin = {}, ro._lin
+
+    def tap(x, P_, name):
+        y = lin(x, P_, name)
+        taps.setdefault(name, []).append((x, y))
+        return y
+    monkeypatch.setattr(ro, "_lin", tap)
+    out, valid, w, cc = ro.aggregate(P, ro.AggCfg(use_nearest=V), c(g["sampled_color"]), rw2c, c(g["sampled_dir"]), c(g["sampled_conf"]),
+                                     c(g["sampled_embedding"]), c(g["sampled_xyz_pers"]), c(g["sampled_xyz"]), T(g["sample_pnt_mask"]),
+                                     c(d["sample_loc"]), c(d["sample_loc_w"]), c(d["sample_ray_dirs"]), img_n=c(d["images_nearest"]),
+                                     sample_loc_i_n=c(d["sample_loc_i_n"]), delta_viewdir_n=c(d["delta_viewdir_n"]))
+    monkeypatch.undo()
+    close = lambda x, y, atol=1e-12: np.testing.assert_allclose(x.detach().numpy(), y.detach().numpy(), rtol=1e-10, atol=atol)
+    pidx = T(d["sample_pidx"]).reshape(S, K)
+    loc_w, loc_pers, rays = c(d["sample_loc_w"]).reshape(S, 3), c(d["sample_loc"]).reshape(S, 3), c(d["sample_ray_dirs"]).reshape(S, 3)
+    cam = torch.cat([c(d["campos"]).reshape(3), c(d["camrotc2w"]).reshape(9), rw2c.t().reshape(9)])
+    # weights, clamped confidence, validity
+    rw, rc, rv = h.ref_nbr_weights(c(d["xyz"]), c(d["conf"]), pidx, None, loc_w)
+    assert torch.equal(rv, valid.reshape(-1)) and 0 < int(rv.sum()) < S
+    close(rw, w.reshape(S, K))
+    close(rc, cc.reshape(S, K), atol=1e-11)                  # the oracle clamps at 1e-4, the kernel (and ref) at float32(1e-4)
+    # MLP input rows of the live slots of the valid samples (the oracle's rows, in its order)
+    vlist = rv.nonzero()[:, 0].to(torch.int32)
+    live = pidx[vlist.long()].reshape(-1) >= 0
+    X0, E = h.ref_nbr_features(c(d["xyz"]), c(d["xyz_pers"]), c(d["emb"]), c(d["color"]), c(d["dir"]), pidx, vlist, loc_w, loc_pers, rays, cam)
+    close(X0[live], taps["block1.0"][0][0])
+    close(E[live], taps["block3.0"][0][0][:, 256:])
+    # without the table the perspective coordinates come from cam: equal up to the table's fp32 rounding (x 2^4 in the encoding)
+    X0c, _ = h.ref_nbr_features(c(d["xyz"]), None, c(d["emb"]), c(d["color"]), c(d["dir"]), pidx, vlist, loc_w, loc_pers, rays, cam)
+    close(X0c, X0, atol=1e-5)
+    # density head + weighted K-sum from the oracle's layer-3 outputs (zero rows for masked slots)
+    H = torch.zeros(len(live), 256, dtype=dt)
+    H[live] = torch.nn.functional.leaky_relu(taps["block3.2"][0][1], 0.01)
+    s = vlist.long()
+    sigma, X5, _ = h.ref_alpha_ksum(H, (rw * rc)[s], P["alpha_branch.0.weight"], P["alpha_branch.0.bias"], rays[s] @ cam[12:21].reshape(3, 3))
+    close(X5, taps["color_feature_branch.0"][0][0])
+    close(sigma, out.reshape(S, 4)[s, 0])
+    # pyramid, upsample + truncated lookup, blend
+    img = c(d["images_nearest"])[0]
+    ws = [P[f"aux_block_s{i}.{j}.weight"] for i in (1, 2, 3) for j in (0, 2)]
+    bs = [P[f"aux_block_s{i}.{j}.bias"] for i in (1, 2, 3) for j in (0, 2)]
+    acts = h.ref_pyramid(img, ws, bs)
+    lv = ro.feature_pyramid(img, P)
+    for i in (1, 2, 3):
+        close(acts[2 * i - 1], lv[i])
+    aux, ok = h.ref_image_gather([img] + [acts[i].permute(0, 2, 3, 1) for i in (1, 3, 5)], c(d["sample_loc_i_n"]).reshape(V, S, 2), vlist)
+    assert 0 < int(ok.sum()) < ok.numel()
+    full = ro.full_res_features(lv)
+    for v in range(V):
+        close(aux[v], taps["aux_merge_weight_block.0"][v][0][:, :45])
+        px, py = [t.long() for t in c(d["sample_loc_i_n"]).reshape(V, S, 2)[v, s].to(torch.int32).unbind(-1)]
+        px, py = torch.where(ok[v], px, 0), torch.where(ok[v], py, 0)
+        close(aux[v], full[v][:, py, px].t())
+    sig = torch.stack([torch.sigmoid(taps["aux_merge_weight_block.6"][v][1][:, 0]) for v in range(V)])
+    close(h.ref_blend(aux, sig, ok.to(dt), None), taps["color_mixup_block.0"][0][0][:, 45:])
+    x = torch.randn(50, 6, dtype=dt)
+    close(h.ref_pos_enc(x, 5), ro.pos_enc(x, 5))
+    close(h.ref_view_enc(x[:, :3], 4), ro.pos_enc(x[:, :3], 4, ori=True)[:, 3:])
